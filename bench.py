@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the hot path (contract: see DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 metric  : SE3 Exp+Log Mops/s (1 op = one se3->SE3 Exp plus one SE3->se3 Log on one element)
 workload: BASELINE.json configs[1] — batch 10^6, fp32, per GPU (weak scaling, no data-path collective)
@@ -13,6 +13,8 @@ legs    : LM step/s (PoseInv, reprojection at 1e6 / 1e7 / 2e8 residual rows, pos
           Msamples/s through the public API, each with its own roofline object (bench_legs.py).
 e2e     : same metric through the public API (pp.se3(...).Exp().Log()) with pinned HOST buffers,
           H2D and D2H copies inside the timed region.
+outputs : --dump-outputs DIR writes rank 0's last timed step as DIR/exp_SE3.npy (n, 7) and DIR/log_se3.npy (n, 6),
+          fp32, 52 MB in all; the inputs are seeded, so two builds can be compared output for output.
 The reference arm (--impl reference) times the torch-CPU port of the reference's Exp/Log op
 sequence (oracle/torch_port.py) on all host cores, on a bounded sample of the same workload.
 """
@@ -161,7 +163,7 @@ def run_ours(args):
     ys = [torch.empty(n, 6, device=dev) for _ in range(ring)]
     footprint = ring * n * (24 + 28 + 24)
     f_exp, f_log = _C.fn("b200_se3_exp_fwd_f32"), _C.fn("b200_SE3_log_fwd_f32")
-    K, W = max(1, args.steps), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
 
     def step(j, sp, which=3):
         if which & 1:
@@ -215,6 +217,10 @@ def run_ours(args):
         ms = timed_region(graphs, K)
         barrier(world)
         regions.append(max_over_ranks(ms, world, dev))
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        last = (K - 1) % ring                  # timed_region replays the ring slots in order
+        outputs = {"exp_SE3": Xs[last].cpu().numpy(), "log_se3": ys[last].cpu().numpy()}
     # keep the GPU busy long enough for nvidia-smi to see clocks under load (a 0.4 ms region is shorter than one sample)
     t_end = time.perf_counter() + 0.35
     while time.perf_counter() < t_end:
@@ -291,6 +297,11 @@ def run_ours(args):
     cpu = cpu_baseline(sample_batches=10) if (rank == 0 and world == 1 and not args.no_cpu) else None
     import bench_legs
     legs = bench_legs.run(args, rank, world, dev, peak)
+    if outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if rank == 0:
         cfg = base_config(world)
         cfg.update({"launch": "CUDA graphs: K // 8 trips of an 8-step graph + K % 8 single-step graphs", "timed_regions": REGIONS,
@@ -405,7 +416,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-large", dest="no_large", action="store_true", help="skip the 2e8-residual LM leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed Exp+Log step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
