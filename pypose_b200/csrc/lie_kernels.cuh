@@ -123,8 +123,16 @@ template <class Op, int S, int OS, int THREADS = kThreads, int EPT = 1> struct T
   static constexpr int BYTES = (S * IN_WORDS + OS * OUT_WORDS) * (int)sizeof(T) + 8 * S;
 };
 
+// Timeline probe hooks (tools/variants/trace.cu defines them; the shipped library expands them to nothing).
+// B200POSE_TRACE(k) runs in stream_kernel_tma at k = 0 entry, 1 after griddepcontrol.wait, 2 tile 0 landed,
+// 3 last store issued (thread 0), 4 exit.
+#ifndef B200POSE_TRACE
+#define B200POSE_TRACE(k)
+#endif
+
 // THREADS threads per CTA, EPT rows per thread per tile (rows tid, tid + THREADS, ...), S input / OS output stages.
-template <class Op, int S, int OS, int THREADS = kThreads, int EPT = 1>
+// PF: tiles of the CTA's inputs hinted into L2 before the dependency wait (0 = none).
+template <class Op, int S, int OS, int THREADS = kThreads, int EPT = 1, int PF = S>
 __global__ void __launch_bounds__(THREADS) stream_kernel_tma(StreamParams<typename Op::T, Op::NIN, Op::NOUT> p) {
   using T = typename Op::T;
   using L = TmaLayout<Op, S, OS, THREADS, EPT>;
@@ -140,15 +148,31 @@ __global__ void __launch_bounds__(THREADS) stream_kernel_tma(StreamParams<typena
   const int ntiles = begin < end ? (int)((end - begin + TILE - 1) / TILE) : 0;
   const int tid = threadIdx.x;
 
-  // Programmatic dependent launch: let the next kernel in the stream start its launch/prologue now, and
-  // hold our own first global access until the previous kernel has completed and flushed.
+  B200POSE_TRACE(0);
+  // Programmatic dependent launch: let the next kernel in the stream start its launch/prologue now (its CTAs take
+  // the SM slots this grid leaves free), and hold our own first load until the previous kernel has completed and
+  // flushed.
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   if (tid == 0) {
 #pragma unroll
     for (int s = 0; s < S; ++s) mbar_init(&full[s], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    // Warm L2 with the first PF tiles of every input while the previous grid drains.  Safe before the wait: a
+    // prefetch is only a hint, never the value a load returns; L2 is the device's point of coherence, and every
+    // load below is issued after griddepcontrol.wait, so it sees all writes of the previous grid (the Exp -> Log
+    // chain reads what the previous launch wrote).  [begin, pf_end) lies within [0, n) and both ends are multiples
+    // of 4 rows, so addresses and sizes are 16-byte multiples like the bulk loads'.  At most PF tiles per CTA:
+    // bounded by the grid's ring footprint, so a large batch cannot flush L2 with hints.
+    if (PF > 0 && begin < end) {
+      const long long pf_end = end - begin > (long long)PF * TILE ? begin + (long long)PF * TILE : end;
+      const uint32_t rows = (uint32_t)(pf_end - begin);
+      bulk_prefetch_l2(p.in[0] + begin * Op::DI0, rows * Op::DI0 * sizeof(T));
+      if (Op::NIN > 1) bulk_prefetch_l2(p.in[Op::NIN > 1 ? 1 : 0] + begin * Op::DI1, rows * Op::DI1 * sizeof(T));
+      if (Op::NIN > 2) bulk_prefetch_l2(p.in[Op::NIN > 2 ? 2 : 0] + begin * Op::DI2, rows * Op::DI2 * sizeof(T));
+    }
   }
   asm volatile("griddepcontrol.wait;" ::: "memory");
+  B200POSE_TRACE(1);
   __syncthreads();
 
   const int last_cnt = ntiles ? (int)(end - begin - (long long)(ntiles - 1) * TILE) : 0;
@@ -182,6 +206,7 @@ __global__ void __launch_bounds__(THREADS) stream_kernel_tma(StreamParams<typena
     T* out1 = out0 + TILE * Op::DO0;
 
     mbar_wait(&full[s], parity);
+    if (i == 0) B200POSE_TRACE(2);
 #pragma unroll
     for (int e = 0; e < EPT; ++e) {
       const int row = tid + e * THREADS;
@@ -206,11 +231,15 @@ __global__ void __launch_bounds__(THREADS) stream_kernel_tma(StreamParams<typena
       if (Op::NOUT > 1) bulk_s2g(p.out[Op::NOUT > 1 ? 1 : 0] + base * Op::DO1, out1, cnt * Op::DO1 * sizeof(T));
       bulk_commit();
       if (i + S < ntiles) issue_load(i + S, s);
+      if (i == ntiles - 1) B200POSE_TRACE(3);
     }
     if (++s == S) { s = 0; parity ^= 1; }
     if (++os == OS) os = 0;
   }
-  if (tid == 0) bulk_wait_all();
+  // Only the shared-memory reads of the stores must finish before the CTA frees its slot; their global writes are
+  // covered by grid completion, which is what the next kernel's griddepcontrol.wait (or stream order) waits for.
+  if (tid == 0) bulk_wait_read<0>();
+  B200POSE_TRACE(4);
 }
 
 constexpr int kMaxDevices = 64;
@@ -282,11 +311,11 @@ inline int stream_max_ctas_per_sm() {
   return v;
 }
 
-template <class Op, int S, int OS, int THREADS = kThreads, int EPT = 1>
+template <class Op, int S, int OS, int THREADS = kThreads, int EPT = 1, int PF = S>
 int launch_stream_tma(const typename Op::T* const* in, typename Op::T* const* out, long long n, cudaStream_t stream) {
   using T = typename Op::T;
   using L = TmaLayout<Op, S, OS, THREADS, EPT>;
-  auto kern = stream_kernel_tma<Op, S, OS, THREADS, EPT>;
+  auto kern = stream_kernel_tma<Op, S, OS, THREADS, EPT, PF>;
   static thread_local int occ_dev[kMaxDevices] = {};
   int& occ = occ_dev[current_device_slot()];
   if (occ == 0) {
@@ -301,7 +330,11 @@ int launch_stream_tma(const typename Op::T* const* in, typename Op::T* const* ou
   p.vec_ok = 1;
   p.n = n;
   long long tiles = (n + L::TILE - 1) / L::TILE;
-  long long slots = (long long)device_info().sms * occ;
+  // With PDL, a shell whose SM holds >= 6 CTAs takes half of them per launch, so the next launch's CTAs are resident
+  // (and warm L2 with their first tiles) while this one drains, instead of each boundary waiting for the whole grid
+  // to exit.  With fewer slots (fp64, multi-operand rows) half a machine keeps too few bytes in flight: full grid.
+  const int per_sm = stream_pdl() && occ >= 6 ? occ / 2 : occ;
+  long long slots = (long long)device_info().sms * per_sm;
   long long grid = tiles < slots ? tiles : slots;
   long long chunk = (n + grid - 1) / grid;
   chunk = (chunk + 3) & ~3LL;

@@ -32,12 +32,15 @@ __device__ __forceinline__ void bulk_s2g(void* gdst, const void* smem_src, uint3
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
                ::"l"(gdst), "r"(smem_u32(smem_src)), "r"(bytes) : "memory");
 }
+// L2 prefetch hint (SASS UBLKPF.L2): no destination, no completion mechanism, never the value a load returns.
+__device__ __forceinline__ void bulk_prefetch_l2(const void* gsrc, uint32_t bytes) {
+  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gsrc), "r"(bytes) : "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void bulk_wait_read() {
   asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
 }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }

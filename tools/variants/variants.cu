@@ -1,22 +1,23 @@
-// DEV ONLY (not part of the package): alternative tilings of the v2 shell for the headline kernels, built into
+// DEV ONLY (not part of the package): candidate configurations of the v2 shell for the headline kernels, built into
 // tools/variants/libvariants.so by tools/variants/build.sh and timed by tools/variants/ab.py.
+// NAME = <op>_<dtype>_s<S>o<OS>_pf<PF>: S input / OS output stages, PF tiles hinted into L2 before the dependency
+// wait.  The grid policy is the shipped launcher's (B200POSE_PDL / B200POSE_CTAS_PER_SM apply).
 #include "lie_kernels.cuh"
 using namespace b200pose;
-#define VAR(NAME, OPT, S, OS, TH, EPT)                                                          \
-  extern "C" __attribute__((visibility("default"))) int NAME(const float* i0, float* o0, long long n, void* st) { \
-    const float* in[1] = {i0}; float* out[1] = {o0};                                           \
-    return launch_stream_tma<OPT<SE3g, float>, S, OS, TH, EPT>(in, out, n, (cudaStream_t)st);  \
+#define VAR(OPN, OPT, CT, SFX, S, OS, PF)                                                                          \
+  extern "C" __attribute__((visibility("default"))) int OPN##_##SFX##_s##S##o##OS##_pf##PF(                        \
+      const CT* i0, CT* o0, long long n, void* st) {                                                               \
+    const CT* in[1] = {i0}; CT* out[1] = {o0};                                                                     \
+    return launch_stream_tma<OPT<SE3g, CT>, S, OS, kThreads, 1, PF>(in, out, n, (cudaStream_t)st);                \
   }
-VAR(exp_s3o2_t256_e1, OpExpFwd, 3, 2, 256, 1)
-VAR(exp_s2o2_t256_e1, OpExpFwd, 2, 2, 256, 1)
-VAR(exp_s2o2_t256_e2, OpExpFwd, 2, 2, 256, 2)
-VAR(exp_s3o2_t128_e2, OpExpFwd, 3, 2, 128, 2)
-VAR(exp_s2o2_t512_e1, OpExpFwd, 2, 2, 512, 1)
-VAR(exp_s3o2_t128_e1, OpExpFwd, 3, 2, 128, 1)
-VAR(exp_s4o2_t128_e1, OpExpFwd, 4, 2, 128, 1)
-VAR(exp_s3o3_t256_e1, OpExpFwd, 3, 3, 256, 1)
-VAR(log_s3o2_t256_e1, OpLogFwd, 3, 2, 256, 1)
-VAR(log_s2o2_t256_e2, OpLogFwd, 2, 2, 256, 2)
-VAR(log_s3o2_t128_e2, OpLogFwd, 3, 2, 128, 2)
-VAR(log_s3o2_t128_e1, OpLogFwd, 3, 2, 128, 1)
-VAR(log_s2o2_t512_e1, OpLogFwd, 2, 2, 512, 1)
+#define PAIR(CT, SFX, S, OS, PF) VAR(exp, OpExpFwd, CT, SFX, S, OS, PF) VAR(log, OpLogFwd, CT, SFX, S, OS, PF)
+PAIR(float, f32, 3, 2, 0)    // no hint
+PAIR(float, f32, 3, 2, 3)    // the shipped fp32 configuration
+PAIR(float, f32, 3, 2, 6)
+PAIR(float, f32, 3, 1, 3)
+PAIR(float, f32, 3, 1, 6)
+PAIR(float, f32, 2, 1, 2)
+PAIR(float, f32, 4, 1, 4)
+PAIR(double, f64, 2, 2, 0)
+PAIR(double, f64, 2, 2, 2)   // the shipped fp64 configuration
+PAIR(double, f64, 2, 1, 2)
