@@ -8,7 +8,7 @@ import os
 
 import torch
 
-from ._optable import lie_symbols, lm_symbols, scan_symbols
+from ._optable import lie_symbols, lm_symbols, scan_symbols, knn_symbols, KNN_QUERIES
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libb200pose.so")
@@ -43,6 +43,8 @@ def _bind(symbol, n_in, n_out, extra=()):
 _LIE = {s: (ct, ins, outs) for s, ct, ins, outs, _ in lie_symbols()}
 _LM = {s: args for s, args, _ in lm_symbols()}
 _SCAN = {s: args for s, args, _ in scan_symbols()}
+_KNN = {s: args for s, args, _ in knn_symbols()}
+_QUERY = {s: (ret, args) for s, ret, args, _ in KNN_QUERIES}
 _CT = {"double": ctypes.c_double, "int": ctypes.c_int, "long long": ctypes.c_longlong}
 
 
@@ -57,10 +59,16 @@ def fn(symbol):
             f.restype = ctypes.c_int
             f.argtypes = [ctypes.c_void_p if "*" in t else _CT[t] for t, _, _ in _LM[symbol]] + \
                 [ctypes.c_longlong, ctypes.c_void_p]
-        elif symbol in _SCAN:
+        elif symbol in _SCAN or symbol in _KNN:
             f = getattr(lib(), symbol)
             f.restype = ctypes.c_int
-            f.argtypes = [ctypes.c_void_p if "*" in t else _CT[t] for t, _, _ in _SCAN[symbol]] + [ctypes.c_void_p]
+            args = _SCAN[symbol] if symbol in _SCAN else _KNN[symbol]
+            f.argtypes = [ctypes.c_void_p if "*" in t else _CT[t] for t, _, _ in args] + [ctypes.c_void_p]
+        elif symbol in _QUERY:
+            ret, args = _QUERY[symbol]
+            f = getattr(lib(), symbol)
+            f.restype = _CT[ret]
+            f.argtypes = [ctypes.c_void_p if "*" in t else _CT[t] for t, _, _ in args]
         else:
             raise B200PoseError(f"unknown C-ABI symbol {symbol}")
         _fns[symbol] = f

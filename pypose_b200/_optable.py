@@ -443,3 +443,48 @@ def scan_symbols():
     for base, args, cite in SCAN_OPS:
         for sfx, ct in DTYPES.items():
             yield f"{base}_{sfx}", [(t.replace("REAL", ct), n, c) for t, n, c in args], cite
+
+
+# ----------------------------------------------------------------------------------------------
+# k-nearest neighbours and the ICP correspondence step (csrc/knn.cu): (symbol base, args, citation); REAL as above.
+# Splits and workspace size come from b200_knn_plan.
+# ----------------------------------------------------------------------------------------------
+KNN_OPS = [
+    ("b200_knn",
+     [("const REAL*", "ref", "(B|1, N1, D) queries, row-major"), ("long long", "ref_bstride", "elements between batches, 0: one cloud for all"),
+      ("const REAL*", "nbr", "(B|1, N2, D) neighbours"), ("long long", "nbr_bstride", "elements between batches, 0: one cloud for all"),
+      ("long long", "B", "batches"), ("long long", "N1", "queries per batch"), ("long long", "N2", "neighbours per batch, < 2^31"),
+      ("int", "D", "1..8"), ("int", "k", "1..min(32, N2)"), ("int", "ord", "1, 2, or 0 for inf"),
+      ("int", "largest", "1: the k furthest"), ("long long", "splits", "S from b200_knn_plan"),
+      ("void*", "ws", "b200_knn_plan bytes of scratch, or NULL when splits == 1"),
+      ("REAL*", "values", "(B, N1, k) ord-norm distances, sorted"), ("long long*", "indices", "(B, N1, k) neighbour indices")],
+     "knn, pypose/function/geometry.py:228-313 (norm of the broadcast difference + topk), streamed without the "
+     "(N1, N2, D) difference tensor; ties keep the lower neighbour index"),
+    ("b200_icp_moments",
+     [("const REAL*", "src", "(B|1, N1, 3) source points"), ("long long", "src_bstride", "elements between batches, 0: one cloud for all"),
+      ("const REAL*", "tgt", "(B|1, N2, 3) target points"), ("long long", "tgt_bstride", "elements between batches, 0: one cloud for all"),
+      ("const REAL*", "pose", "(B, 7) current SE3 estimate T applied to src"), ("long long", "B", "batches"),
+      ("long long", "N1", "source points"), ("long long", "N2", "target points, 1 .. 2^31 - 1"), ("int", "ord", "1, 2, or 0 for inf"),
+      ("long long", "splits", "S from b200_knn_plan with k = 1"), ("void*", "ws", "b200_knn_plan bytes, or NULL when splits == 1"),
+      ("double*", "moments", "(B, 17) accumulated (zeroed by the caller): count, sum T s (3), sum t (3), "
+                             "sum t (T s)^T row-major (9), sum of nearest-neighbour distances")],
+     "one iteration of ICP.forward, pypose/module/icp.py: knn(T source, target, k=1) + gather + the moments of "
+     "svdtf (geometry.py:315-358), without materialising the transformed cloud"),
+]
+
+
+# host-side queries of csrc/knn.cu: (symbol, return type, [(ctype, name, comment)], description)
+KNN_QUERIES = [
+    ("b200_knn_plan", "long long",
+     [("long long", "B", "batches"), ("long long", "N1", "queries per batch"), ("long long", "N2", "neighbours per batch"),
+      ("int", "k", "results per query"), ("int", "elem_size", "4 or 8"), ("int", "sms", "multiprocessors of the device"),
+      ("long long*", "splits", "out: S, the number of N2 chunks (1 = no split)")],
+     "Number of N2 splits for a search of B x N1 queries over N2 neighbours, chosen from the shapes; returns the "
+     "workspace bytes that split needs (0 when S == 1)"),
+]
+
+
+def knn_symbols():
+    for base, args, cite in KNN_OPS:
+        for sfx, ct in DTYPES.items():
+            yield f"{base}_{sfx}", [(t.replace("REAL", ct), n, c) for t, n, c in args], cite

@@ -4,3 +4,4 @@ from .ba import BundleAdjustment
 from .imu_preintegrator import IMUPreintegrator
 from .loss import GeodesicLoss, geodesic_loss
 from .pnp import EPnP
+from .icp import ICP

@@ -1,1 +1,2 @@
 from .io import read_bal, read_g2o
+from .stepper import ReduceToBason
